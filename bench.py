@@ -7,12 +7,14 @@ horizon: LQ approximation + projection + Riccati + filter line search), policy e
 trot gait schedule, horizon 1.0 s / dt 0.01 (100 intervals + event nodes), batch 8192 robots PER GPU (weak scaling),
 synthetic 24-DoF states (SURVEY §8d), fp64.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl b200|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl b200|reference] [--dump-outputs DIR]
 
 `value`   device-resident: inputs already in HBM, CUDA events on the launch stream, max over ranks.
 `e2e`     the same tick through the C-ABI host call qmb200_tick with pinned HOST buffers (H2D of the observation,
           schedule and targets, D2H of the 54-vector inside the timed region).
 `--impl reference` times the CPU restatement of the reference path (oracle/, all host threads) on a bounded sample.
+`--dump-outputs DIR` writes what the last timed step returned as DIR/<name>.npy (see dump_outputs).  The inputs are seeded
+          per robot, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -178,6 +180,24 @@ def run_reference(args, rank, world):
                       "cpu_baseline": info, "e2e": {"value": info["value"], "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}}))
 
 
+DUMP_LIMIT = 64 << 20      # bytes --dump-outputs may write in all
+
+
+def dump_outputs(path, arrays):
+    """Each array as <path>/<name>.npy in float64 (int32 status words convert exactly).  When they would exceed DUMP_LIMIT, every array keeps the same
+    fraction of its rows (robots), drawn with a fixed seed so that equal row counts keep equal rows, and <name>_rows.npy lists the rows kept."""
+    arrays = {k: np.asarray(v, dtype=np.float64) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT:
+        frac = (DUMP_LIMIT - 4096) / (total + 8 * sum(a.shape[0] for a in arrays.values()))   # the row lists and .npy headers count too
+        for k in list(arrays):
+            n = arrays[k].shape[0]; rows = np.sort(np.random.default_rng(0).choice(n, max(1, int(n * frac)), replace=False))
+            arrays[k] = arrays[k][rows]; arrays[k + "_rows"] = rows.astype(np.float64)
+    os.makedirs(path, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), a)
+
+
 KEYS = ("t0", "x0", "n_events", "event_times", "modes", "n_target", "target_times", "target_states")
 ST_NAMES = {1: "iter_cap", 2: "overflow", 4: "nan", 8: "not_pd", 16: "no_step", 32: "converged", 64: "neg_dt"}
 
@@ -232,6 +252,13 @@ class TickLoop:
         ag = self.ev[0].elapsed_time(self.ev[1]) if self.ev else 0.0
         return e0.elapsed_time(e1) / steps, self.solver.launch_count - l0, ag
 
+    def outputs(self):
+        """What the last step handed its caller: the 54-vector and status word per robot, and the gathered torque rows when step() gathers them."""
+        out = {"cmd": self.cmd_d.cpu().numpy(), "status": self.st_d.cpu().numpy()}
+        if self.world > 1 or self.perm_d is not None:
+            out["torque_all"] = self.all_d.cpu().numpy()
+        return out
+
     def flagged(self):
         st = self.st_d.cpu().numpy(); mpc = (st >> 8) & 0xFF; wbcs = st & 0xFF; out = {}
         for bit, name in ST_NAMES.items():
@@ -252,7 +279,7 @@ def side_workload(args, q, torch, dev, local, stream):
     peaks, peak_src = measured_peaks(); n_int = int(round(HORIZON / DT)); W = args.workload
     if W == "mixed":
         B = args.batch if args.batch != UNIT_BATCH else 2048; loop = TickLoop(q, torch, dev, local, stream, B, np.arange(3 * B, 4 * B), 5, 1, 0)
-        ms, launches, _ = loop.timed(args.steps, args.warmup, dev); ab = algorithmic_bytes(n_int)["total"]
+        ms, launches, _ = loop.timed(args.steps, args.warmup, dev); ab = algorithmic_bytes(n_int)["total"]; outputs = loop.outputs
         out = {"workload": "configs[4] per-GPU share: mixed stance / trot / flying-trot batch, full MPC+WBC tick", "batch": B, "flagged": loop.flagged()}
     elif W == "mpc":
         B = args.batch if args.batch != UNIT_BATCH else 1024; solver = q.Solver(batch=B, device=local, dt=DT, time_horizon=HORIZON)
@@ -264,7 +291,7 @@ def side_workload(args, q, torch, dev, local, stream):
         torch.cuda.synchronize(dev); l0 = solver.launch_count; e0 = torch.cuda.Event(enable_timing=True); e1 = torch.cuda.Event(enable_timing=True); e0.record()
         for _ in range(args.steps):
             step()
-        e1.record(); torch.cuda.synchronize(dev); ms = e0.elapsed_time(e1) / args.steps; launches = solver.launch_count - l0; ab = 15840 * n_int + 2328
+        e1.record(); torch.cuda.synchronize(dev); ms = e0.elapsed_time(e1) / args.steps; launches = solver.launch_count - l0; ab = 15840 * n_int + 2328; outputs = solver.mpc_get_solution
         out = {"workload": "configs[1]: batched MPC only (one SQP iteration), state 30 / input 30, horizon 100, stance", "batch": B, "l2": "stage buffer %.1f GB >> 126 MB L2" % (B * solver.nmax * 1484 * 8 / 1e9)}
     else:
         B = args.batch if args.batch != UNIT_BATCH else 4096; solver = q.Solver(batch=B, device=local)
@@ -280,7 +307,10 @@ def side_workload(args, q, torch, dev, local, stream):
             if i >= args.warmup:
                 pairs.append((a, b))
         torch.cuda.synchronize(dev); ms = float(np.mean([a.elapsed_time(b) for a, b in pairs])); launches = args.steps; ab = 1856
+        outputs = lambda: {"cmd": cmd.cpu().numpy(), "status": st.cpu().numpy()}
         out = {"workload": "configs[2]: batched WBC only (3-level HoQp, 36 decision variables, 54 outputs), stance", "batch": B, "l2": "256 MB written between launches (L2 flush), timed per launch with CUDA events", "flagged_robots": int(np.count_nonzero(st.cpu().numpy()))}
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outputs())
     ach = ab * B / (ms * 1e-3) / 1e9
     print(json.dumps({"metric": "robot_iters_per_s", "value": B / (ms * 1e-3), "unit": "robot-iterations/s of the named workload", "n_gpus": 1, "steps": args.steps, "warmup": args.warmup, "ms_per_step": ms, "higher_is_better": True,
                       "scaling": "weak", "vs_baseline": None, "dtype": "f64", "data": "synthetic", "config": out, "gpu_launches": int(launches),
@@ -296,7 +326,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true"); ap.add_argument("--no-e2e", action="store_true"); ap.add_argument("--no-extras", action="store_true", help="skip the strong-scaling and configs[4] records")
     ap.add_argument("--solver", default="sqp", choices=["sqp", "ipm", "ddp"], help="MPC solver variant (qmb200_mpc_set_solver); the BASELINE metric is quoted on sqp, the controller's solver")
     ap.add_argument("--chunks", type=int, default=PIPELINE_CHUNKS, help="robot ranges run as concurrent stream chains inside one tick")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned as DIR/<name>.npy (float64, at most 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl b200)")
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1"))
     if args.impl == "reference":
         run_reference(args, rank, world); return
@@ -322,6 +357,8 @@ def main():
     sampler = ClockSampler(local); sampler.start(); time.sleep(0.15)
     ms_local, launches, ag_ms = loop.timed(args.steps, 0, dev, dist)
     clocks = sampler.finish()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, loop.outputs())
     ms = parallel.max_over_ranks(ms_local, dev); ag_ms = parallel.max_over_ranks(ag_ms, dev)
     value = (B * world / UNIT_BATCH) / (ms * 1e-3)
     flagged = loop.flagged()

@@ -2,7 +2,7 @@
 
 Every other test feeds the derived files under assets/ (tools/make_assets.py: comments stripped, the unused ddp / ipm / rollout blocks and the visual /
 collision / gazebo elements dropped).  Here byte-identical copies of the reference's task.info, reference.info, gait.info and robot.urdf
-(tests/fixtures/ref_inputs/, md5 pinned below) go through the same parser — host only, no GPU — and must produce the same model + settings block,
+(tests/golden/ref_inputs/, md5 pinned below) go through the same parser — host only, no GPU — and must produce the same model + settings block,
 byte for byte, that is replicated to every GPU; the oracle's own parser must agree on the quantities both expose."""
 import ctypes as C
 import hashlib
@@ -13,7 +13,7 @@ import numpy as np
 from qm_control_b200 import _lib
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-REF = os.path.join(HERE, "fixtures", "ref_inputs")
+REF = os.path.join(HERE, "golden", "ref_inputs")
 MD5 = {"task.info": "47e417bf5dea44b5bcb85f43dc792c4f", "reference.info": "650b9c7f61c223c013eed33f58389054", "gait.info": "ad3bcc5374db06f6ff8b20eba56a0b59",
        "robot.urdf": "2438ccb67bb3b37781c4cd7f6bf56919"}   # of the files in skywoodsz/qm_control @ 67247bb
 

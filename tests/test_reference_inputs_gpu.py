@@ -1,4 +1,4 @@
-"""A handle created from byte-identical copies of the reference's own task.info / reference.info / robot.urdf (tests/fixtures/ref_inputs/) solves the same
+"""A handle created from byte-identical copies of the reference's own task.info / reference.info / robot.urdf (tests/golden/ref_inputs/) solves the same
 tick, bit for bit, as the handle every other test creates from the derived assets/ files (tests/test_reference_inputs_cpu.py checks the parsed constants)."""
 import os
 
@@ -6,7 +6,7 @@ import numpy as np
 import pytest
 
 pytestmark = pytest.mark.gpu
-REF = os.path.join(os.path.dirname(os.path.abspath(__file__)), "fixtures", "ref_inputs")
+REF = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ref_inputs")
 
 
 def test_tick_on_the_reference_files_is_bit_identical_to_the_assets():

@@ -11,7 +11,7 @@ import pytest
 from _parity import MPC_TOL, assert_traj
 
 pytestmark = pytest.mark.gpu
-REF_TASK = os.path.join(os.path.dirname(os.path.abspath(__file__)), "fixtures", "ref_inputs", "task.info")
+REF_TASK = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ref_inputs", "task.info")
 
 
 def _block(name):
