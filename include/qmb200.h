@@ -131,6 +131,26 @@ int qmb200_mpc_get_solution(qmb200_handle* h, int32_t* n_nodes, double* node_tim
 int qmb200_policy_eval(qmb200_handle* h, const double* t /*[B]*/, double* x_des /*[B][30]*/, double* u_des /*[B][30]*/, int32_t* mode /*[B]*/);
 int qmb200_policy_eval_dev(qmb200_handle* h, const double* t, double* x_des, double* u_des, int32_t* mode, void* cuda_stream);
 
+/* ---- feedback policy: useFeedbackPolicy of the ddp{} / sqp{} / ipm{} blocks (task.info:61,89,107).  When it is on, OCS2 stores the solve as an
+ *      ocs2::LinearController u = uff(t) + K(t) x and MPC_MRT_Interface::evaluatePolicy(currentTime, currentState, ...) (QMController.cpp:141) reacts to the
+ *      measured state between two MPC updates.  K_k = Px_k + Pu_k K~_k is the derivative of the QP's optimal input step at node k with respect to the state
+ *      step (the projected Riccati gain mapped back to the full input), uff_k = u*_k - K_k x*_k on the stored solution; a pre-event node and the last node
+ *      repeat the bias and gain of the node before them; bias and gain are interpolated separately on the node times.  Robots whose last solve carries
+ *      QMB200_ST_NOT_PD, _NAN, _OVERFLOW or _NEG_DT keep the feed-forward policy (zero gain).  After qmb200_mpc_set_solution / qmb200_mpc_reset there is no
+ *      controller until the next solve.  With the switch on, qmb200_tick evaluates at (t_eval, x0) and qmb200_update at (t_obs, x_obs); with it off every
+ *      entry point evaluates the feed-forward policy, as before.  qmb200_create reads sqp.useFeedbackPolicy, qmb200_mpc_set_solver the chosen block's key. */
+int qmb200_mpc_set_feedback_policy(qmb200_handle* h, int32_t on);
+int qmb200_mpc_get_feedback_policy(const qmb200_handle* h, int32_t* on);
+/* MPC_MRT_Interface::evaluatePolicy(currentTime, currentState, → optimizedState, optimizedInput, plannedMode): x_des and mode as qmb200_policy_eval; u_des of the
+ * feedback policy at x (switch off: identical to qmb200_policy_eval, x is not read) */
+int qmb200_policy_eval_state(qmb200_handle* h, const double* t /*[B]*/, const double* x /*[B][30]*/, double* x_des /*[B][30]*/, double* u_des /*[B][30]*/, int32_t* mode /*[B]*/);
+int qmb200_policy_eval_state_dev(qmb200_handle* h, const double* t, const double* x, double* x_des, double* u_des, int32_t* mode, void* cuda_stream);
+/* ocs2::LinearController of the last solve (timeStamp = the node times of qmb200_mpc_get_solution) for robots [b0, b0 + count): biasArray, gainArray (row = input,
+ * column = state) per node, zero past the robot's node count; feedback[r] = 0 where the robot has the feed-forward controller (gain zero, bias = u*).
+ * The host variant exports through a device scratch of at most 256 MB. */
+int qmb200_mpc_get_controller(qmb200_handle* h, int32_t b0, int32_t count, double* bias /*[count][NMAX][30]*/, double* gain /*[count][NMAX][30][30]*/, int32_t* feedback /*[count]*/);
+int qmb200_mpc_get_controller_dev(qmb200_handle* h, int32_t b0, int32_t count, double* bias, double* gain, int32_t* feedback, void* cuda_stream);
+
 /* ---- one controller tick on the device: mpc_solve → policy_eval(t_eval) → wbc_update, torque buffer out.
  *      Host-pointer version: observation in, cmd out (the e2e path bench.py times). */
 int qmb200_tick(qmb200_handle* h, const double* t0, const double* x0, const int32_t* n_events, const double* event_times, const int32_t* mode_sequence,

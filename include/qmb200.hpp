@@ -105,6 +105,9 @@ class HierarchicalMpcWbc : public WbcBase {
 // ocs2::ModeSchedule / ocs2::TargetTrajectories in the solver's flat layout (one robot)
 struct ModeSchedule { std::vector<double> eventTimes; std::vector<int32_t> modeSequence; };          // modeSequence.size() == eventTimes.size() + 1
 struct TargetTrajectories { std::vector<double> timeTrajectory; std::vector<vector_t> stateTrajectory; };   // states of 37 = 30 + EE pose
+// ocs2::LinearController of one robot: u(t, x) = bias(t) + gain(t) x, piecewise linear in t on timeStamp (gainArray[k]: 30 x 30 row-major, row = input).
+// feedback == false: the feed-forward controller (no solve since the last set_solution / reset, or the last QP had no defined gain).
+struct LinearController { std::vector<double> timeStamp; std::vector<vector_t> biasArray, gainArray; bool feedback = false; };
 struct PrimalSolution { std::vector<double> timeTrajectory; std::vector<int32_t> postEventAnnotation; std::vector<vector_t> stateTrajectory, inputTrajectory; int32_t status = 0; double stepSize = 0.0; };
 
 // SqpMpc + MPC_MRT_Interface for one robot (QMController.cpp:286-312): run() = MPC_BASE::run (sqp.sqpIteration SQP iterations, warm started), evaluatePolicy()
@@ -135,6 +138,24 @@ class SqpMpc {
   void evaluatePolicy(scalar_t currentTime, vector_t& optimizedState, vector_t& optimizedInput, size_t& plannedMode) {
     optimizedState.resize(QMB200_NX); optimizedInput.resize(QMB200_NU); int32_t mode = 0;
     solver_->check(qmb200_policy_eval(solver_->get(), &currentTime, optimizedState.data(), optimizedInput.data(), &mode), "SqpMpc::evaluatePolicy"); plannedMode = static_cast<size_t>(mode);
+  }
+  // the reference's signature: with setFeedbackPolicy(true) the input reacts to currentState (u = uff(t) + K(t) x), otherwise the overload above
+  void evaluatePolicy(scalar_t currentTime, const vector_t& currentState, vector_t& optimizedState, vector_t& optimizedInput, size_t& plannedMode) {
+    if (currentState.size() != QMB200_NX) throw std::runtime_error("SqpMpc::evaluatePolicy: wrong state size");
+    optimizedState.resize(QMB200_NX); optimizedInput.resize(QMB200_NU); int32_t mode = 0;
+    solver_->check(qmb200_policy_eval_state(solver_->get(), &currentTime, currentState.data(), optimizedState.data(), optimizedInput.data(), &mode), "SqpMpc::evaluatePolicy"); plannedMode = static_cast<size_t>(mode);
+  }
+  // useFeedbackPolicy of the solver block (task.info:61,89,107); setSolver() re-reads the chosen block's value
+  void setFeedbackPolicy(bool on) { solver_->check(qmb200_mpc_set_feedback_policy(solver_->get(), on ? 1 : 0), "SqpMpc::setFeedbackPolicy"); }
+  // PrimalSolution::controllerPtr_ as a LinearController (MPC_MRT_Interface::getPolicy)
+  LinearController getLinearController() {
+    const int nmax = solver_->maxNodes(); int32_t n = 0, fb = 0; std::vector<double> t(nmax), bias((size_t)nmax * QMB200_NU), gain((size_t)nmax * QMB200_NU * QMB200_NX);
+    solver_->check(qmb200_mpc_get_solution(solver_->get(), &n, t.data(), nullptr, nullptr, nullptr, nullptr, nullptr), "SqpMpc::getLinearController");
+    solver_->check(qmb200_mpc_get_controller(solver_->get(), 0, 1, bias.data(), gain.data(), &fb), "SqpMpc::getLinearController");
+    LinearController c; c.feedback = fb != 0;
+    for (int k = 0; k < n; ++k) { c.timeStamp.push_back(t[k]); c.biasArray.emplace_back(bias.begin() + (size_t)k * QMB200_NU, bias.begin() + (size_t)(k + 1) * QMB200_NU);
+      c.gainArray.emplace_back(gain.begin() + (size_t)k * QMB200_NU * QMB200_NX, gain.begin() + (size_t)(k + 1) * QMB200_NU * QMB200_NX); }
+    return c;
   }
 
  private:

@@ -33,7 +33,7 @@ struct qmb200_handle {
   std::string err, task_file;   // task_file: qmb200_mpc_set_solver re-reads the sqp{} / ipm{} / ddp{} block
   int64_t launches = 0;
   // staging for the host-pointer API
-  double *d_xdes = nullptr, *d_udes = nullptr, *d_rbd = nullptr, *d_period = nullptr, *d_time = nullptr, *d_cmd = nullptr, *d_input_last = nullptr, *d_teval = nullptr;
+  double *d_xdes = nullptr, *d_udes = nullptr, *d_rbd = nullptr, *d_period = nullptr, *d_time = nullptr, *d_cmd = nullptr, *d_input_last = nullptr, *d_teval = nullptr, *d_xeval = nullptr;
   int32_t *d_mode = nullptr, *d_status = nullptr, *d_wbc_diag = nullptr;   // d_wbc_diag: per-robot WBC iteration counts (qmb200_wbc_get_diagnostics), kept out of the status word
   MpcBuffers mpc;   // device buffers of the MPC path (kernels/mpc_api.cuh)
   std::vector<void*> allocs;
@@ -49,6 +49,11 @@ struct qmb200_handle {
   double hw_delay = 0.0; double *hw_ring_cmd = nullptr, *hw_ring_stamp = nullptr; int32_t* hw_ring_state = nullptr;   // QMHWSim command-delay FIFO
   void* comm = nullptr; int comm_ranks = 0, comm_rank = 0; double* d_send = nullptr;   // NCCL communicator of this handle (capi_comm.inc) and the packed torque rows
   int chunks = 1; cudaStream_t cs[MAX_CHUNKS] = {nullptr}; cudaEvent_t fork_ev = nullptr, join_ev[MAX_CHUNKS] = {nullptr};
+  // useFeedbackPolicy of the active solver block; has_controller: the stage records / projected gains belong to the stored solution (a solve ran since the
+  // last set_solution / reset).  Policy evaluation is feedback only when both hold.
+  bool feedback_policy = false, has_controller = false;
+  double *d_ctrl_bias = nullptr, *d_ctrl_gain = nullptr; int32_t* d_ctrl_fb = nullptr; int ctrl_rows = 0;   // bounded scratch of qmb200_mpc_get_controller
+  bool feedback_on() const { return feedback_policy && has_controller; }
 };
 
 namespace {
@@ -75,6 +80,7 @@ int qmb200_create(const qmb200_config* cfg, qmb200_handle** out) {
     h->target_prm.com_height = ref.number("comHeight"); h->target_prm.target_displacement_velocity = ref.number("targetDisplacementVelocity");
     h->target_prm.target_rotation_velocity = ref.number("targetRotationVelocity"); h->target_prm.time_to_target = task.number("mpc.timeHorizon");
     for (int j = 0; j < NJ; ++j) h->target_prm.default_joint_state[j] = h->hm.default_joint_state[j];
+    h->feedback_policy = task.boolean("sqp.useFeedbackPolicy", false);   // the handle starts with SqpMpc (QMController.cpp:287-288)
   } catch (const std::exception& e) { g_create_error = e.what(); delete h; return -2; }
   if (cfg->time_horizon > 0) h->hm.dev.time_horizon = cfg->time_horizon;
   if (cfg->dt > 0) h->hm.dev.dt = cfg->dt;
@@ -90,7 +96,7 @@ int qmb200_create(const qmb200_config* cfg, qmb200_handle** out) {
   if (wbc_configure_device() != 0 || mpc_configure_device() != 0) { g_create_error = std::string("qmb200_create: cudaFuncSetAttribute failed: ") + cudaGetErrorString(cudaGetLastError()); qmb200_destroy(h); return -3; }
   const size_t B = (size_t)h->B;
   bool ok = dalloc(h, &h->d_model, 1) && dalloc(h, &h->d_xdes, B * NX) && dalloc(h, &h->d_udes, B * NU) && dalloc(h, &h->d_rbd, B * QMB200_RBD) && dalloc(h, &h->d_period, B) &&
-            dalloc(h, &h->d_time, B) && dalloc(h, &h->d_cmd, B * QMB200_CMD) && dalloc(h, &h->d_input_last, B * NU) && dalloc(h, &h->d_mode, B) && dalloc(h, &h->d_status, B) && dalloc(h, &h->d_teval, B) && dalloc(h, &h->d_wbc_diag, B);
+            dalloc(h, &h->d_time, B) && dalloc(h, &h->d_cmd, B * QMB200_CMD) && dalloc(h, &h->d_input_last, B * NU) && dalloc(h, &h->d_mode, B) && dalloc(h, &h->d_status, B) && dalloc(h, &h->d_teval, B) && dalloc(h, &h->d_xeval, B * NX) && dalloc(h, &h->d_wbc_diag, B);
   if (ok) { std::string merr; ok = mpc_alloc(h->mpc, h->B, h->nmax, merr, h->allocs, h->stream); if (!ok) h->err = merr; }
   if (!ok) { g_create_error = h->err; qmb200_destroy(h); return -4; }
   cudaMemcpyAsync(h->d_model, &h->hm.dev, sizeof(DevModel), cudaMemcpyHostToDevice, h->stream);

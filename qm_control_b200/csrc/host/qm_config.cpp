@@ -49,6 +49,11 @@ InfoFile::InfoFile(const std::string& path) {
 }
 double InfoFile::number(const std::string& key) const { auto it = values_.find(key); if (it == values_.end()) throw std::runtime_error("INFO key missing: " + key); return std::stod(it->second); }
 std::string InfoFile::text(const std::string& key) const { auto it = values_.find(key); if (it == values_.end()) throw std::runtime_error("INFO key missing: " + key); return it->second; }
+bool InfoFile::boolean(const std::string& key, bool fallback) const {
+  auto it = values_.find(key); if (it == values_.end()) return fallback;
+  if (it->second == "true" || it->second == "1") return true; if (it->second == "false" || it->second == "0") return false;
+  throw std::runtime_error("INFO key " + key + ": not a boolean: " + it->second);
+}
 std::vector<double> InfoFile::matrix(const std::string& key, int rows, int cols) const {
   std::vector<double> m((size_t)rows * cols, 0.0); auto it = nodes_.find(key); if (it == nodes_.end()) throw std::runtime_error("INFO matrix missing: " + key);
   const double scaling = number(key + ".scaling", 1.0);

@@ -21,6 +21,8 @@ class InfoFile {
   double number(const std::string& key) const;
   double number(const std::string& key, double fallback) const { return has(key) ? number(key) : fallback; }
   std::string text(const std::string& key) const;
+  // boolean leaf as ocs2::loadData::loadPtreeValue<bool> reads it ("true" / "false", "1" / "0"); a missing key gives `fallback`, any other value throws
+  bool boolean(const std::string& key, bool fallback) const;
   // ocs2::loadData::loadEigenMatrix semantics ("(i,j) value" entries times optional "scaling")
   std::vector<double> matrix(const std::string& key, int rows, int cols) const;
   // "[i] value" children of a node, in index order

@@ -67,6 +67,12 @@ int mpc_solve_launch(const DevModel* mdl, const DevModel& host_mdl, MpcBuffers& 
 double measure_fp64_peak(cudaStream_t stream);
 // evaluatePolicy on m.sol[m.cur]; returns kernels launched
 int mpc_policy_eval_launch(const MpcBuffers& m, const double* t, double* x_des, double* u_des, int32_t* mode, cudaStream_t stream, int b0 = 0, int b1 = -1);
+// evaluatePolicy(t, x): with `feedback` the LinearController of the last solve (stage record + projected gains, u = uff(t) + K(t) x), otherwise exactly
+// mpc_policy_eval_launch (x is not read).  One launch either way; returns kernels launched
+int mpc_policy_launch(const DevModel* mdl, const MpcBuffers& m, bool feedback, const double* t, const double* x, double* x_des, double* u_des, int32_t* mode, cudaStream_t stream, int b0 = 0, int b1 = -1);
+// dense LinearController of robots [b0, b0 + count): bias [count][nmax][30], gain [count][nmax][30][30] (row = input), feedback flag [count]; `valid` false (no
+// solve since the last set_solution / reset) exports the feed-forward controller
+int mpc_controller_export_launch(const DevModel* mdl, const MpcBuffers& m, bool valid, int b0, int count, double* bias, double* gain, int32_t* feedback, cudaStream_t stream);
 // input fix-up after loading a solution from the host (inputs at pre-event / last nodes)
 int mpc_fixup_launch(const MpcBuffers& m, cudaStream_t stream);
 

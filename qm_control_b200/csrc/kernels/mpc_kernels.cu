@@ -1113,6 +1113,81 @@ __global__ void mpc_policy_eval_kernel(int b0, int B, int nmax, MpcSolutionDev s
 }
 
 // =====================================================================================================
+// Feedback policy (useFeedbackPolicy of the ddp / sqp / ipm blocks): the LinearController u = uff(t) + K(t) x of the last solve
+// [upstream ocs2_oc multiple_shooting::toPrimalSolution with feedback, recalled]:
+//   K_k = Px_k + Pu_k K~_k (remapProjectedGain), uff_k = u*_k - K_k x*_k on the solution after the step; a pre-event node and the last node repeat the bias and
+//   gain of the node before them.  The controller is never materialised: the solve's stage record and projected gains stay untouched until the next solve, and
+//   rollout_input() with alpha = 0 evaluates u*_s + (Px_s + Pu_s K~_s)(x - x*_s) = uff_s + K_s x from them.
+// Robots whose last QP has no defined K~ (not positive definite, NaN, overflow, non-positive interval) keep the feed-forward policy.
+constexpr int MST_NO_FEEDBACK = MST_OVERFLOW | MST_NAN | MST_NOT_PD | MST_NEG_DT;
+// node whose bias and gain node k of an n-node solution uses, -1 when there is none (zero gain, bias = u*_k)
+__device__ __forceinline__ int controller_node(const int32_t* __restrict__ ge, int n, int k) {
+  int s = k; while (s > 0 && (s == n - 1 || ge[s] == 1)) --s;
+  return (s >= n - 1 || ge[s] == 1) ? -1 : s;
+}
+// One warp per robot: the two bracketing nodes' projected gains (4.9 KB each) and record tails (3.4 KB each) are staged in shared memory with coalesced loads,
+// then lanes 0 / 1 evaluate one node each with rollout_input() on the staged copy, and the lanes of the inputs blend the two with alpha.
+constexpr int PF_WARPS = 2;
+struct PolicySmem { double K[2][GAIN_DBL]; double tail[2][TAIL_DBL]; double dx[2][NX]; double u[2][NU]; };
+__global__ void __launch_bounds__(32 * PF_WARPS) mpc_policy_feedback_kernel(const DevModel* __restrict__ mdl, int b0, int B, int nmax, MpcSolutionDev sol, const double* __restrict__ stage,
+                                                                           const double* __restrict__ gains, const int32_t* __restrict__ status, const int32_t* __restrict__ n_events,
+                                                                           const double* __restrict__ event_times, const int32_t* __restrict__ modes, const double* __restrict__ tq,
+                                                                           const double* __restrict__ xq, double* __restrict__ x_des, double* __restrict__ u_des, int32_t* __restrict__ mode_out) {
+  __shared__ PolicySmem s_pol[PF_WARPS];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31; const int b = b0 + blockIdx.x * PF_WARPS + warp; if (b >= B) return;
+  PolicySmem& sm = s_pol[warp];
+  const int n = sol.n_nodes[b]; const double* gt = sol.t + (size_t)b * nmax; const int32_t* ge = sol.event + (size_t)b * nmax; const double t = tq[b];
+  int idx; double a; time_segment(gt, n, t, idx, a); const int i2 = (idx + 1 < n) ? idx + 1 : idx;
+  const double* gx = sol.x + (size_t)b * nmax * NX; const double* gu = sol.u + (size_t)b * nmax * NU;
+  if (lane < NX) x_des[(size_t)b * NX + lane] = a * gx[(size_t)idx * NX + lane] + (1.0 - a) * gx[(size_t)i2 * NX + lane];
+  if (lane == 0) mode_out[b] = mode_at_time(event_times + (size_t)b * EMAX, modes + (size_t)b * (EMAX + 1), clamp_events(n_events[b]), t);
+  if (status[b] & MST_NO_FEEDBACK) {   // the feed-forward arithmetic of mpc_policy_eval_kernel
+    if (lane < NU) u_des[(size_t)b * NU + lane] = a * gu[(size_t)idx * NU + lane] + (1.0 - a) * gu[(size_t)i2 * NU + lane];
+    return;
+  }
+  const int src0 = controller_node(ge, n, idx), src1 = controller_node(ge, n, i2);
+#pragma unroll
+  for (int j = 0; j < 2; ++j) {
+    const int s = j ? src1 : src0; if (s < 0) continue;   // warp-uniform
+    const size_t node = (size_t)b * nmax + s; const double* kg = gains + node * GAIN_DBL; const double* tl = stage + node * STAGE_DBL + ST_TAIL;
+    for (int e = lane; e < GAIN_DBL; e += 32) sm.K[j][e] = kg[e];
+    for (int e = lane; e < TAIL_DBL; e += 32) sm.tail[j][e] = tl[e];
+    if (lane < NX) sm.dx[j][lane] = xq[(size_t)b * NX + lane] - gx[(size_t)s * NX + lane];
+  }
+  __syncwarp();
+  if (lane < 2) {
+    const int s = lane ? src1 : src0;
+    if (s >= 0) rollout_input(sm.tail[lane], sm.K[lane], gu + (size_t)s * NU, sm.dx[lane], 0.0, pack_leg_foot(mdl), sm.u[lane]);
+    else { const int k = lane ? i2 : idx; for (int c = 0; c < NU; ++c) sm.u[lane][c] = gu[(size_t)k * NU + c]; }
+  }
+  __syncwarp();
+  if (lane < NU) u_des[(size_t)b * NU + lane] = a * sm.u[0][lane] + (1.0 - a) * sm.u[1][lane];
+}
+
+// Dense LinearController of robots [b0, b0 + count): one warp per (robot, node).  Lane j < 30 evaluates column j of K_k as rollout_input() of the unit vector e_j
+// around a zero nominal input, lane 30 the bias u*_s + K_s (0 - x*_s).  Robots without a controller (or with `valid` false) get a zero gain and bias = u*_k.
+__global__ void __launch_bounds__(32) mpc_controller_export_kernel(const DevModel* __restrict__ mdl, int b0, int nmax, MpcSolutionDev sol, const double* __restrict__ stage, const double* __restrict__ gains,
+                                                                  const int32_t* __restrict__ status, int valid, double* __restrict__ bias, double* __restrict__ gain, int32_t* __restrict__ feedback) {
+  const int r = blockIdx.x, k = blockIdx.y, lane = threadIdx.x; const int b = b0 + r;
+  const int n = sol.n_nodes[b]; const bool fb = valid && !(status[b] & MST_NO_FEEDBACK);
+  if (k == 0 && lane == 0) feedback[r] = fb ? 1 : 0;
+  const int32_t* ge = sol.event + (size_t)b * nmax; const double* gx = sol.x + (size_t)b * nmax * NX; const double* gu = sol.u + (size_t)b * nmax * NU;
+  double* bo = bias + ((size_t)r * nmax + k) * NU; double* go = gain + ((size_t)r * nmax + k) * NU * NX;
+  const int s = (fb && k < n) ? controller_node(ge, n, k) : -1;
+  if (s < 0) {
+    for (int e = lane; e < NU * NX; e += 32) go[e] = 0.0;
+    if (lane < NU) bo[lane] = (k < n) ? gu[(size_t)k * NU + lane] : 0.0;
+    return;
+  }
+  if (lane > NX) return;
+  const size_t node = (size_t)b * nmax + s; double dxv[NX], zero[NU], un[NU];
+  for (int i = 0; i < NX; ++i) { dxv[i] = (lane < NX) ? (i == lane ? 1.0 : 0.0) : -gx[(size_t)s * NX + i]; zero[i] = 0.0; }
+  rollout_input(stage + node * STAGE_DBL + ST_TAIL, gains + node * GAIN_DBL, lane < NX ? zero : gu + (size_t)s * NU, dxv, 0.0, pack_leg_foot(mdl), un);
+  if (lane < NX) { for (int i = 0; i < NU; ++i) go[(size_t)i * NX + lane] = un[i]; }
+  else { for (int i = 0; i < NU; ++i) bo[i] = un[i]; }
+}
+
+// =====================================================================================================
 bool mpc_alloc(MpcBuffers& m, int B, int nmax, std::string& err, std::vector<void*>& allocs, cudaStream_t stream) {
   m.B = B; m.nmax = nmax; m.cur = 0;
   if (SETUP_WARPS * ((setup_smem_per_warp(nmax) + 15) & ~(size_t)15) > 200 * 1024) { err = "max_nodes too large for the grid staging of the setup kernel (limit ~1000 nodes)"; return false; }
@@ -1165,6 +1240,17 @@ int mpc_solve_launch(const DevModel* mdl, const DevModel& hm, MpcBuffers& m, con
 int mpc_policy_eval_launch(const MpcBuffers& m, const double* t, double* x_des, double* u_des, int32_t* mode, cudaStream_t stream, int b0, int b1) {
   if (b1 < 0) b1 = m.B; if (b1 <= b0) return 0;
   mpc_policy_eval_kernel<<<(b1 - b0 + 3) / 4, 128, 0, stream>>>(b0, b1, m.nmax, m.sol[m.cur], m.n_events, m.event_times, m.modes, t, x_des, u_des, mode);
+  return 1;
+}
+int mpc_policy_launch(const DevModel* mdl, const MpcBuffers& m, bool feedback, const double* t, const double* x, double* x_des, double* u_des, int32_t* mode, cudaStream_t stream, int b0, int b1) {
+  if (!feedback) return mpc_policy_eval_launch(m, t, x_des, u_des, mode, stream, b0, b1);
+  if (b1 < 0) b1 = m.B; if (b1 <= b0) return 0;
+  mpc_policy_feedback_kernel<<<(b1 - b0 + PF_WARPS - 1) / PF_WARPS, 32 * PF_WARPS, 0, stream>>>(mdl, b0, b1, m.nmax, m.sol[m.cur], m.stage, m.gains, m.status, m.n_events, m.event_times, m.modes, t, x, x_des, u_des, mode);
+  return 1;
+}
+int mpc_controller_export_launch(const DevModel* mdl, const MpcBuffers& m, bool valid, int b0, int count, double* bias, double* gain, int32_t* feedback, cudaStream_t stream) {
+  if (count <= 0) return 0;
+  mpc_controller_export_kernel<<<dim3(count, m.nmax), 32, 0, stream>>>(mdl, b0, m.nmax, m.sol[m.cur], m.stage, m.gains, m.status, valid ? 1 : 0, bias, gain, feedback);
   return 1;
 }
 int mpc_fixup_launch(const MpcBuffers& m, cudaStream_t stream) { mpc_fixup_kernel<<<m.B, 32, 0, stream>>>(m.B, m.nmax, m.sol[m.cur]); return 1; }

@@ -191,6 +191,32 @@ class Solver:
         self._chk(self.lib.qmb200_policy_eval(self.h, _p(t), _p(xd), _p(ud), _p(mode)), "qmb200_policy_eval")
         return xd, ud, mode
 
+    def mpc_set_feedback_policy(self, on=True):
+        """useFeedbackPolicy: evaluate the LinearController u = uff(t) + K(t) x of the last solve instead of the feed-forward policy (include/qmb200.h)."""
+        self._chk(self.lib.qmb200_mpc_set_feedback_policy(self.h, 1 if on else 0), "qmb200_mpc_set_feedback_policy")
+
+    def mpc_get_feedback_policy(self):
+        v = C.c_int32(); self._chk(self.lib.qmb200_mpc_get_feedback_policy(self.h, C.byref(v)), "qmb200_mpc_get_feedback_policy"); return bool(v.value)
+
+    def policy_eval_state(self, t, x):
+        """MPC_MRT_Interface::evaluatePolicy(t, x) → (x_des, u_des, mode); with the switch off identical to policy_eval(t)."""
+        B = self.batch; t = _f64(t, (B,)); x = _f64(x, (B, NX)); xd = np.empty((B, NX)); ud = np.empty((B, NU)); mode = np.empty(B, dtype=np.int32)
+        self._chk(self.lib.qmb200_policy_eval_state(self.h, _p(t), _p(x), _p(xd), _p(ud), _p(mode)), "qmb200_policy_eval_state")
+        return xd, ud, mode
+
+    def policy_eval_state_dev(self, t, x, x_des, u_des, mode, stream=None):
+        self._chk(self.lib.qmb200_policy_eval_state_dev(self.h, _p(t), _p(x), _p(x_des), _p(u_des), _p(mode), C.c_void_p(stream) if stream else None), "qmb200_policy_eval_state_dev")
+
+    def mpc_get_controller(self, b0=0, count=None):
+        """LinearController of robots [b0, b0 + count) → dict(bias[count, NMAX, 30], gain[count, NMAX, 30, 30] (row = input), feedback[count])."""
+        count = self.batch - b0 if count is None else int(count); N = self.nmax
+        out = dict(bias=np.zeros((count, N, NU)), gain=np.zeros((count, N, NU, NX)), feedback=np.zeros(count, dtype=np.int32))
+        self._chk(self.lib.qmb200_mpc_get_controller(self.h, int(b0), count, _p(out["bias"]), _p(out["gain"]), _p(out["feedback"])), "qmb200_mpc_get_controller")
+        return out
+
+    def mpc_get_controller_dev(self, b0, count, bias, gain, feedback, stream=None):
+        self._chk(self.lib.qmb200_mpc_get_controller_dev(self.h, int(b0), int(count), _p(bias), _p(gain), _p(feedback), C.c_void_p(stream) if stream else None), "qmb200_mpc_get_controller_dev")
+
     def tick(self, prob, t_eval, rbd, period):
         B = self.batch; a = self._prob(prob); t_eval = _f64(t_eval, (B,)); rbd = _f64(rbd, (B, RBD)); period = _f64(period, (B,))
         cmd = np.empty((B, CMD)); status = np.empty(B, dtype=np.int32)

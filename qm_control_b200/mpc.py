@@ -16,6 +16,16 @@ class SqpMpc:
         """MPC_BASE::run(t0, x0) for every robot; prob as in Solver.mpc_solve. Returns the PrimalSolution arrays."""
         return self.solver.mpc_solve(prob)
 
-    def evaluatePolicy(self, t):
-        """MPC_MRT_Interface::evaluatePolicy → (optimizedState, optimizedInput, plannedMode)."""
-        return self.solver.policy_eval(t)
+    def setFeedbackPolicy(self, on=True):
+        """useFeedbackPolicy: the policy becomes the LinearController u = uff(t) + K(t) x of the last solve."""
+        self.solver.mpc_set_feedback_policy(on)
+
+    def evaluatePolicy(self, t, x=None):
+        """MPC_MRT_Interface::evaluatePolicy(currentTime, currentState) → (optimizedState, optimizedInput, plannedMode).  Without a state the
+        feed-forward policy is evaluated."""
+        return self.solver.policy_eval(t) if x is None else self.solver.policy_eval_state(t, x)
+
+    def getLinearController(self, b0=0, count=None):
+        """ocs2::LinearController of the last solve: dict(timeStamp[count, NMAX], biasArray, gainArray, feedback) (see Solver.mpc_get_controller)."""
+        c = self.solver.mpc_get_controller(b0, count); sol = self.solver.mpc_get_solution(); n = len(c["feedback"])
+        return dict(timeStamp=sol["t"][b0:b0 + n], n_nodes=sol["n_nodes"][b0:b0 + n], biasArray=c["bias"], gainArray=c["gain"], feedback=c["feedback"])
