@@ -151,6 +151,21 @@ int qmb200_policy_eval_state_dev(qmb200_handle* h, const double* t, const double
 int qmb200_mpc_get_controller(qmb200_handle* h, int32_t b0, int32_t count, double* bias /*[count][NMAX][30]*/, double* gain /*[count][NMAX][30][30]*/, int32_t* feedback /*[count]*/);
 int qmb200_mpc_get_controller_dev(qmb200_handle* h, int32_t b0, int32_t count, double* bias, double* gain, int32_t* feedback, void* cuda_stream);
 
+/* ---- value function: createValueFunction of the sqp{} / ipm{} blocks (OCS2 default false; the shipped task.info does not set it).  When it is on, the solve
+ *      keeps what SqpSolver / IpmSolver::extractValueFunction keep after the QP of the robot's last iteration: per node k (node 0, event nodes and the terminal
+ *      node included) dfdxx_k = P_k and dfdx_k = p_k - P_k xbar_k, where P_k, p_k are the Riccati cost-to-go of the state step dx_k in full state coordinates and
+ *      xbar is that QP's linearization trajectory (the iterate before the step).  A robot that converged early keeps the value function of its last QP.
+ *      getValueFunction(t, x) returns f = 0, dfdxx and dfdx interpolated linearly on the node times (the (index, alpha) of qmb200_policy_eval, clamped before the
+ *      first and past the last node), then dfdx += dfdxx x.  valid[b] = 1 only when the last solve ran with the switch on, robot b's QP was factorised (no
+ *      QMB200_ST_NOT_PD, _NAN, _OVERFLOW, _NEG_DT) and no qmb200_mpc_set_solution / qmb200_mpc_reset followed; elsewhere the outputs are zero.
+ *      qmb200_create reads sqp.createValueFunction, qmb200_mpc_set_solver the chosen block's key; DDP turns the switch off (GaussNewtonDDP::getValueFunction has
+ *      a different contract) and refuses it.  The records take NMAX * 3,968 B per robot, allocated when the switch is first turned on; if that allocation fails
+ *      the call returns an error and the switch stays off.  With the switch off the solve is unchanged. */
+int qmb200_mpc_set_value_function(qmb200_handle* h, int32_t on);
+int qmb200_mpc_get_value_function(const qmb200_handle* h, int32_t* on);
+int qmb200_value_function(qmb200_handle* h, const double* t /*[B]*/, const double* x /*[B][30]*/, double* dfdx /*[B][30]*/, double* dfdxx /*[B][30][30]*/, int32_t* valid /*[B]*/);
+int qmb200_value_function_dev(qmb200_handle* h, const double* t, const double* x, double* dfdx, double* dfdxx, int32_t* valid, void* cuda_stream);
+
 /* ---- one controller tick on the device: mpc_solve → policy_eval(t_eval) → wbc_update, torque buffer out.
  *      Host-pointer version: observation in, cmd out (the e2e path bench.py times). */
 int qmb200_tick(qmb200_handle* h, const double* t0, const double* x0, const int32_t* n_events, const double* event_times, const int32_t* mode_sequence,

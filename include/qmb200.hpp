@@ -108,6 +108,8 @@ struct TargetTrajectories { std::vector<double> timeTrajectory; std::vector<vect
 // ocs2::LinearController of one robot: u(t, x) = bias(t) + gain(t) x, piecewise linear in t on timeStamp (gainArray[k]: 30 x 30 row-major, row = input).
 // feedback == false: the feed-forward controller (no solve since the last set_solution / reset, or the last QP had no defined gain).
 struct LinearController { std::vector<double> timeStamp; std::vector<vector_t> biasArray, gainArray; bool feedback = false; };
+// ocs2::ScalarFunctionQuadraticApproximation of the value function at (t, x): f (0, as SqpSolver::getValueFunction leaves it), dfdx (30), dfdxx (30 x 30 row-major)
+struct ValueFunction { scalar_t f = 0.0; vector_t dfdx, dfdxx; };
 struct PrimalSolution { std::vector<double> timeTrajectory; std::vector<int32_t> postEventAnnotation; std::vector<vector_t> stateTrajectory, inputTrajectory; int32_t status = 0; double stepSize = 0.0; };
 
 // SqpMpc + MPC_MRT_Interface for one robot (QMController.cpp:286-312): run() = MPC_BASE::run (sqp.sqpIteration SQP iterations, warm started), evaluatePolicy()
@@ -147,6 +149,17 @@ class SqpMpc {
   }
   // useFeedbackPolicy of the solver block (task.info:61,89,107); setSolver() re-reads the chosen block's value
   void setFeedbackPolicy(bool on) { solver_->check(qmb200_mpc_set_feedback_policy(solver_->get(), on ? 1 : 0), "SqpMpc::setFeedbackPolicy"); }
+  // createValueFunction of the solver block; setSolver() re-reads the chosen block's value (DDP: off, and turning it on throws)
+  void setValueFunction(bool on) { solver_->check(qmb200_mpc_set_value_function(solver_->get(), on ? 1 : 0), "SqpMpc::setValueFunction"); }
+  // SqpSolver::getValueFunction(time, state) (MPC_MRT_Interface::getValueFunction); throws std::runtime_error when there is none, as OCS2 does when
+  // valueFunction_ is empty (switch off at the last solve, set_solution / reset since, or the last QP was not factorised)
+  ValueFunction getValueFunction(scalar_t time, const vector_t& state) {
+    if (state.size() != QMB200_NX) throw std::runtime_error("SqpMpc::getValueFunction: wrong state size");
+    ValueFunction v; v.dfdx.resize(QMB200_NX); v.dfdxx.resize((size_t)QMB200_NX * QMB200_NX); int32_t valid = 0;
+    solver_->check(qmb200_value_function(solver_->get(), &time, state.data(), v.dfdx.data(), v.dfdxx.data(), &valid), "SqpMpc::getValueFunction");
+    if (!valid) throw std::runtime_error("SqpMpc::getValueFunction: no value function (createValueFunction off at the last solve, no solve since set_solution / reset, or the QP was not factorised)");
+    return v;
+  }
   // PrimalSolution::controllerPtr_ as a LinearController (MPC_MRT_Interface::getPolicy)
   LinearController getLinearController() {
     const int nmax = solver_->maxNodes(); int32_t n = 0, fb = 0; std::vector<double> t(nmax), bias((size_t)nmax * QMB200_NU), gain((size_t)nmax * QMB200_NU * QMB200_NX);

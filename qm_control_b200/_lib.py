@@ -38,7 +38,8 @@ SYMBOLS = ["qmb200_create", "qmb200_destroy", "qmb200_last_error", "qmb200_get_d
            "qmb200_observation_update", "qmb200_observation_update_dev", "qmb200_target_trajectories", "qmb200_target_trajectories_dev", "qmb200_initial_ee_target",
            "qmb200_control_law", "qmb200_control_law_dev", "qmb200_set_arm_gains", "qmb200_hw_write", "qmb200_hw_write_dev", "qmb200_hw_set_delay", "qmb200_update", "qmb200_update_dev",
            "qmb200_debug_model_blob", "qmb200_comm_get_unique_id", "qmb200_comm_init", "qmb200_comm_destroy", "qmb200_comm_info", "qmb200_allgather_torque", "qmb200_gait_bin_permutation", "qmb200_set_pipeline", "qmb200_set_profiling", "qmb200_collect_kernel_times", "qmb200_get_kernel_times", "qmb200_get_flow_kernel_time", "qmb200_measure_fp64_peak",
-           "qmb200_mpc_set_feedback_policy", "qmb200_mpc_get_feedback_policy", "qmb200_policy_eval_state", "qmb200_policy_eval_state_dev", "qmb200_mpc_get_controller", "qmb200_mpc_get_controller_dev"]
+           "qmb200_mpc_set_feedback_policy", "qmb200_mpc_get_feedback_policy", "qmb200_policy_eval_state", "qmb200_policy_eval_state_dev", "qmb200_mpc_get_controller", "qmb200_mpc_get_controller_dev",
+           "qmb200_mpc_set_value_function", "qmb200_mpc_get_value_function", "qmb200_value_function", "qmb200_value_function_dev"]
 
 _lib = None
 

@@ -54,6 +54,10 @@ struct qmb200_handle {
   bool feedback_policy = false, has_controller = false;
   double *d_ctrl_bias = nullptr, *d_ctrl_gain = nullptr; int32_t* d_ctrl_fb = nullptr; int ctrl_rows = 0;   // bounded scratch of qmb200_mpc_get_controller
   bool feedback_on() const { return feedback_policy && has_controller; }
+  // createValueFunction of the active solver block (never on with DDP); has_value_function: the last solve ran with it on and no set_solution / reset
+  // followed, so mpc.vf holds that solve's records.  qmb200_value_function reports a robot valid when this holds and its last QP was factorised.
+  bool value_function = false, has_value_function = false;
+  double *d_vf_dfdx = nullptr, *d_vf_dfdxx = nullptr; int32_t* d_vf_valid = nullptr;   // staging of qmb200_value_function
 };
 
 namespace {
@@ -81,6 +85,7 @@ int qmb200_create(const qmb200_config* cfg, qmb200_handle** out) {
     h->target_prm.target_rotation_velocity = ref.number("targetRotationVelocity"); h->target_prm.time_to_target = task.number("mpc.timeHorizon");
     for (int j = 0; j < NJ; ++j) h->target_prm.default_joint_state[j] = h->hm.default_joint_state[j];
     h->feedback_policy = task.boolean("sqp.useFeedbackPolicy", false);   // the handle starts with SqpMpc (QMController.cpp:287-288)
+    h->value_function = task.boolean("sqp.createValueFunction", false);
   } catch (const std::exception& e) { g_create_error = e.what(); delete h; return -2; }
   if (cfg->time_horizon > 0) h->hm.dev.time_horizon = cfg->time_horizon;
   if (cfg->dt > 0) h->hm.dev.dt = cfg->dt;
@@ -98,6 +103,7 @@ int qmb200_create(const qmb200_config* cfg, qmb200_handle** out) {
   bool ok = dalloc(h, &h->d_model, 1) && dalloc(h, &h->d_xdes, B * NX) && dalloc(h, &h->d_udes, B * NU) && dalloc(h, &h->d_rbd, B * QMB200_RBD) && dalloc(h, &h->d_period, B) &&
             dalloc(h, &h->d_time, B) && dalloc(h, &h->d_cmd, B * QMB200_CMD) && dalloc(h, &h->d_input_last, B * NU) && dalloc(h, &h->d_mode, B) && dalloc(h, &h->d_status, B) && dalloc(h, &h->d_teval, B) && dalloc(h, &h->d_xeval, B * NX) && dalloc(h, &h->d_wbc_diag, B);
   if (ok) { std::string merr; ok = mpc_alloc(h->mpc, h->B, h->nmax, merr, h->allocs, h->stream); if (!ok) h->err = merr; }
+  if (ok && h->value_function) ok = dalloc(h, &h->mpc.vf, B * h->nmax * VF_DBL);   // 3,968 B per robot and node
   if (!ok) { g_create_error = h->err; qmb200_destroy(h); return -4; }
   cudaMemcpyAsync(h->d_model, &h->hm.dev, sizeof(DevModel), cudaMemcpyHostToDevice, h->stream);
   if (cudaStreamSynchronize(h->stream) != cudaSuccess) { g_create_error = std::string("qmb200_create: ") + cudaGetErrorString(cudaGetLastError()); qmb200_destroy(h); return -4; }   // buffers zeroed, constants resident before any (user-stream) launch

@@ -39,6 +39,10 @@ constexpr int SI_TYPE = 0, SI_M = 1, SI_NDEP = 2, SI_DEP = 3, SI_FREE = 19, SI_P
 static_assert(STAGE_DBL == 1484 && (ST_BR % 2 == 0) && (ST_Q % 2 == 0) && (ST_TAIL % 2 == 0) && (TAIL_DBL % 2 == 0), "16-byte aligned pieces");
 constexpr int GAIN_DBL = 18 * LDG;       // feedback K (m x 30) with the pitch of its shared-memory target, feedforward k in column 30
 constexpr int ROBOT_DBL = 8;                 // armijo, base cost, base dyn SSE, base eq SSE, |dx|, |du|
+// Value function record of one node (createValueFunction): dfdxx = P_k as a packed lower triangle (entry (r, c), c <= r, at r (r + 1) / 2 + c), then
+// dfdx = p_k - P_k xbar_k (xbar: the linearization trajectory of the QP), padded to an even count
+constexpr int VF_P = 465, VF_DBL = 496;
+static_assert(VF_P == 30 * 31 / 2 && VF_DBL >= VF_P + 30 && VF_DBL % 2 == 0, "value function record");
 
 // PrimalSolution of every robot: node count, node times, event annotation (0 none, 1 pre-event, 2 post-event), x, u
 struct MpcSolutionDev { int32_t* n_nodes = nullptr; double* t = nullptr; int32_t* event = nullptr; double* x = nullptr; double* u = nullptr; };
@@ -52,6 +56,7 @@ struct MpcBuffers {
   double *ddp_trial = nullptr;  // DDP line search: cost and equality SSE of every step length, [B][32][2]
   double *node_rec = nullptr;   // K2a -> K2b: per node the flow-map / constraint / end-effector record (ne::NodeRec, 492 doubles)
   double *stage = nullptr, *gains = nullptr, *dx = nullptr, *du = nullptr, *robot = nullptr, *step_info = nullptr;
+  double *vf = nullptr;         // [B][nmax][VF_DBL] value function of the last QP (createValueFunction), allocated by the handle on first use
   int32_t *stage_i = nullptr, *status = nullptr;
 };
 bool mpc_alloc(MpcBuffers& m, int B, int nmax, std::string& err, std::vector<void*>& allocs, cudaStream_t stream);
@@ -62,7 +67,8 @@ struct MpcProblemDev { const double* t0; const double* x0; const int32_t* n_even
 // One SQP iteration for robots [b0, b1) (4 kernels on `stream`): reads m.sol[m.cur], writes m.sol[1 - m.cur]; the caller
 // flips m.cur after queueing every range.  Returns the number of kernels launched.
 // `ev` (optional, 8 events): [0..4] recorded before K1 and after each of K1, K2 (flow + LQ), K3, K4 for per-kernel timing; [7] between the flow kernel and the LQ kernel.
-int mpc_solve_launch(const DevModel* mdl, const DevModel& host_mdl, MpcBuffers& m, const MpcProblemDev& p, int b0, int b1, cudaStream_t stream, cudaEvent_t* ev = nullptr);
+// `value_fn`: K3 also stores every node's value function into m.vf (which must be allocated); the launch count does not change.
+int mpc_solve_launch(const DevModel* mdl, const DevModel& host_mdl, MpcBuffers& m, const MpcProblemDev& p, int b0, int b1, cudaStream_t stream, cudaEvent_t* ev = nullptr, bool value_fn = false);
 // fp64 FMA throughput microbenchmark (roofline denominator for the compute-bound kernels); returns TFLOP/s
 double measure_fp64_peak(cudaStream_t stream);
 // evaluatePolicy on m.sol[m.cur]; returns kernels launched
@@ -73,6 +79,9 @@ int mpc_policy_launch(const DevModel* mdl, const MpcBuffers& m, bool feedback, c
 // dense LinearController of robots [b0, b0 + count): bias [count][nmax][30], gain [count][nmax][30][30] (row = input), feedback flag [count]; `valid` false (no
 // solve since the last set_solution / reset) exports the feed-forward controller
 int mpc_controller_export_launch(const DevModel* mdl, const MpcBuffers& m, bool valid, int b0, int count, double* bias, double* gain, int32_t* feedback, cudaStream_t stream);
+// getValueFunction(t, x) of every robot: dfdxx [B][30][30] (full, symmetric) and dfdx [B][30] of the stored records interpolated on the node times as
+// mpc_policy_eval_launch interpolates, plus dfdxx x; valid[b] = `valid` and robot b's last QP was factorised.  Zero outputs where valid[b] = 0.  Returns kernels launched
+int mpc_value_function_launch(const MpcBuffers& m, bool valid, const double* t, const double* x, double* dfdx, double* dfdxx, int32_t* valid_out, cudaStream_t stream);
 // input fix-up after loading a solution from the host (inputs at pre-event / last nodes)
 int mpc_fixup_launch(const MpcBuffers& m, cudaStream_t stream);
 

@@ -576,8 +576,14 @@ __device__ __forceinline__ void cfrag_store(double* M, int ld, int i0, int j0, i
 // support position (0..11) of state column j for the leg whose first joint is `first`, -1 outside the support (inverse of sup_col)
 __device__ __forceinline__ int sup_pos(int j, int first) { return j < 6 ? j : ((j >= 9 && j < 12) ? j - 3 : (((unsigned)(j - 12 - first) < 3u) ? 9 + j - 12 - first : -1)); }
 
+// kValueFn (createValueFunction): every node's cost-to-go of dx_k is also stored as a VF_DBL record (mpc_api.cuh) in `vf`, re-centred on the linearization
+// trajectory sol.x (which K4 overwrites only after this kernel): dfdxx_k = P_k, dfdx_k = p_k - P_k xbar_k.  P_{k+1} is complete and read-only at the top of
+// iteration k (both node types) until phase 3 / the event update rewrite column 30, so node k+1 is stored there; node 0 after the sweep.  The false
+// instantiation is the kernel without the stores.
+template <bool kValueFn>
 __global__ void __launch_bounds__(RIC_THREADS, 4) mpc_riccati_kernel(const DevModel* __restrict__ mdl, int b0, int B, int nmax, MpcProblemDev p, MpcSolutionDev sol, const double* __restrict__ stage,
-                                                                  double* __restrict__ gains, double* __restrict__ dxo, double* __restrict__ duo, double* __restrict__ robot, int32_t* __restrict__ status) {
+                                                                  double* __restrict__ gains, double* __restrict__ dxo, double* __restrict__ duo, double* __restrict__ robot, int32_t* __restrict__ status,
+                                                                  double* __restrict__ vf) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   RicSmem& sm = *reinterpret_cast<RicSmem*>(smem_raw);
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, ti = tid >> 2, jb = tid & 3; const int b = b0 + blockIdx.x;
@@ -621,6 +627,19 @@ __global__ void __launch_bounds__(RIC_THREADS, 4) mpc_riccati_kernel(const DevMo
       if (fa >= 12 && fa < 24) { const int j = fa - 12, lg = j / 3, foot = (lfp >> (2 * lg)) & 3; const int pv = si[SI_PIV + foot]; if (pv >= 0) { const int jf = j - 3 * lg; slot = 2 * foot + (jf > pv ? jf - 1 : jf); first = 3 * lg; } }
       sm.srow[tid] = (signed char)slot; sm.sfirst[tid] = (signed char)first; }
   };
+  // value function record of node kk from sm.P (all threads; sm.P must hold P_kk, p_kk and stay unchanged until the caller's next barrier).  Packed entry e
+  // is (r, e - r (r + 1) / 2) with r = floor((sqrt(8e + 1) - 1) / 2): 8e + 1 < 2^24 is exact in fp32 and the correctly rounded square root of a non-square
+  // 8e + 1 stays below the next integer.  dfdx: 4 threads per row as the rollout's K dx
+  auto store_vf = [&](int kk) {
+    double* out = vf + ((size_t)b * nmax + kk) * VF_DBL;
+    for (int e = tid; e < VF_P; e += RIC_THREADS) { const int r = (int)((sqrtf(8.0f * e + 1.0f) - 1.0f) * 0.5f); out[e] = sm.P[r * LDX + e - (r * (r + 1) >> 1)]; }
+    const double* xb = sol.x + ((size_t)b * nmax + kk) * NX; double s = 0.0;
+    if (ti < NX) {
+#pragma unroll
+      for (int v = 0; v < 8; ++v) { const int c = jb * 8 + v; if (c < NX) s = fma(sm.P[ti * LDX + c], xb[c], s); } }
+    s += __shfl_xor_sync(FULL, s, 1); s += __shfl_xor_sync(FULL, s, 2);
+    if (ti < NX && jb == 0) out[VF_P + ti] = sm.P[ti * LDX + NX] - s;
+  };
   // terminal value function and baseline performance
   for (int e = tid; e < NX * NX; e += RIC_THREADS) { const int r = e / NX, c = e - r * NX; sm.P[r * LDX + c] = sgb[(size_t)N * STAGE_DBL + ST_Q + q_row_offset(r > c ? r : c) + (r > c ? c : r)]; }
   if (tid < NX) sm.P[tid * LDX + NX] = sgb[(size_t)N * STAGE_DBL + ST_TAIL + T_q + tid];
@@ -640,6 +659,7 @@ __global__ void __launch_bounds__(RIC_THREADS, 4) mpc_riccati_kernel(const DevMo
     const int type = node_type(k); const int tnext = k > 0 ? node_type(k - 1) : 1;
     if (type == 1) {                                // event node: A = I, no input: p += P b   (b~ of the node is in the tail, which expand-time waited for)
       __syncthreads();                              // P of node k+1 is complete
+      if (kValueFn) store_vf(k + 1);
       if (tid < NX) { double sv = sm.P[tid * LDX + NX]; for (int j = 0; j < NX; ++j) sv = fma(sm.P[tid * LDX + j], sm.tail[T_b + j], sv); sm.tmp[tid] = sv; }
       __syncthreads();
       if (tid < NX) sm.P[tid * LDX + NX] = sm.tmp[tid];
@@ -647,6 +667,7 @@ __global__ void __launch_bounds__(RIC_THREADS, 4) mpc_riccati_kernel(const DevMo
       continue;
     }
     gAB.wait(); if (QMB_TMA) __syncthreads();     // rows 3:12 of A~, B~ have landed; the rebuilt rows and P of node k+1 are visible to everybody
+    if (kValueFn) store_vf(k + 1);
     // ---- phase 1: W = P'A (32x32: warp = 16x16 block; column 30: p + P b~) ; PB = P'B~ (32x24: warp = row tile) ----
     // Rows 24:30 of A~ (arm joint positions) are identity rows with b~ in column 30, rows 24:30 of B~ carry dtw at the arm's own projected columns (the last six
     // free inputs): their contributions to every product of the sweep are copies / scaled copies of rows of P, W, PB and enter through the C fragments, so the
@@ -756,6 +777,7 @@ __global__ void __launch_bounds__(RIC_THREADS, 4) mpc_riccati_kernel(const DevMo
       double c[2][2][2]; cfrag_load<2, 2>(sm.P, LDX, i0, j0, NX, c, g, t); warp_mma<MU, 2, 2, true>(Yb, LDX, i0, Yb, LDX, j0, c, g, t); cfrag_store<2, 2>(sm.P, LDX, i0, j0, NX, c, g, t); }
   }
   __syncthreads();
+  if (kValueFn && !(st & MST_NOT_PD)) store_vf(0);   // the rollout's first copies land in buffer set 0; sm.P (set 1) is rewritten after its first barrier
   // ---- forward rollout: du~ = K dx + k ; dx+ = A~ dx + B~ du~ + b~ ; du = Px dx + Pu du~ + Pe ; armijo = sum q~'dx + r~'du~.  Works on the structured
   //      record directly (no dense A~ / B~): per node four copies - gains, rows 3:12 of A~ and B~, tail - into one of two buffer sets ----
   double armijo = 0.0, dxn2 = 0.0, dun2 = 0.0;
@@ -1188,6 +1210,36 @@ __global__ void __launch_bounds__(32) mpc_controller_export_kernel(const DevMode
 }
 
 // =====================================================================================================
+// Value function (createValueFunction of the sqp / ipm blocks): SqpSolver::getValueFunction(t, x) [upstream ocs2_sqp, recalled] - f = 0, dfdxx and dfdx of
+// the stored records interpolated linearly on the node times (the (index, alpha) of mpc_policy_eval_kernel, clamped outside the horizon), then
+// dfdx += dfdxx x.  One warp per robot: the two bracketing records (7.9 KB) are staged with coalesced loads and blended in place, so the dense dfdxx
+// written out and the one multiplying x are the same numbers; lane r < 30 forms row r of dfdxx x.
+constexpr int VF_WARPS = 4;
+struct VfSmem { double v[2][VF_DBL]; double x[NX]; };
+__global__ void __launch_bounds__(32 * VF_WARPS) mpc_value_function_kernel(int B, int nmax, MpcSolutionDev sol, const double* __restrict__ vf, const int32_t* __restrict__ status, int valid,
+                                                                           const double* __restrict__ tq, const double* __restrict__ xq, double* __restrict__ dfdx, double* __restrict__ dfdxx,
+                                                                           int32_t* __restrict__ valid_out) {
+  __shared__ VfSmem s_vf[VF_WARPS];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31; const int b = blockIdx.x * VF_WARPS + warp; if (b >= B) return;
+  VfSmem& sm = s_vf[warp]; double* Po = dfdxx + (size_t)b * NX * NX; double* go = dfdx + (size_t)b * NX;
+  const int n = sol.n_nodes[b]; const bool ok = valid && n >= 1 && !(status[b] & MST_NO_FEEDBACK);
+  if (lane == 0) valid_out[b] = ok ? 1 : 0;
+  if (!ok) { for (int e = lane; e < NX * NX; e += 32) Po[e] = 0.0; if (lane < NX) go[lane] = 0.0; return; }
+  int idx; double a; time_segment(sol.t + (size_t)b * nmax, n, tq[b], idx, a); const int i2 = (idx + 1 < n) ? idx + 1 : idx;
+  const double* r0 = vf + ((size_t)b * nmax + idx) * VF_DBL; const double* r1 = vf + ((size_t)b * nmax + i2) * VF_DBL;
+  for (int e = lane; e < VF_P + NX; e += 32) { sm.v[0][e] = r0[e]; sm.v[1][e] = r1[e]; }
+  if (lane < NX) sm.x[lane] = xq[(size_t)b * NX + lane];
+  __syncwarp();
+  for (int e = lane; e < VF_P + NX; e += 32) sm.v[0][e] = a * sm.v[0][e] + (1.0 - a) * sm.v[1][e];
+  __syncwarp();
+  const double* V = sm.v[0];
+  for (int e = lane; e < NX * NX; e += 32) { const int r = e / NX, c = e - r * NX; Po[e] = (c <= r) ? V[(r * (r + 1) >> 1) + c] : V[(c * (c + 1) >> 1) + r]; }
+  if (lane < NX) { double s = V[VF_P + lane];
+    for (int c = 0; c < NX; ++c) s = fma((c <= lane) ? V[(lane * (lane + 1) >> 1) + c] : V[(c * (c + 1) >> 1) + lane], sm.x[c], s);
+    go[lane] = s; }
+}
+
+// =====================================================================================================
 bool mpc_alloc(MpcBuffers& m, int B, int nmax, std::string& err, std::vector<void*>& allocs, cudaStream_t stream) {
   m.B = B; m.nmax = nmax; m.cur = 0;
   if (SETUP_WARPS * ((setup_smem_per_warp(nmax) + 15) & ~(size_t)15) > 200 * 1024) { err = "max_nodes too large for the grid staging of the setup kernel (limit ~1000 nodes)"; return false; }
@@ -1204,11 +1256,12 @@ int mpc_configure_device() {
   if (e == cudaSuccess) e = cudaFuncSetAttribute(mpc_flow_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, FL_SMEM);
   if (e == cudaSuccess) e = cudaFuncSetAttribute(mpc_rollout_trials_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, RO_RPC_MAX * GAIN_DBL * 8);
   if (e == cudaSuccess) e = cudaFuncSetAttribute(mpc_lq_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(sizeof(LqSmem) * LQ_WARPS));
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(mpc_riccati_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(RicSmem));
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(mpc_riccati_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(RicSmem));
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(mpc_riccati_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(RicSmem));
   return (int)e;
 }
 
-int mpc_solve_launch(const DevModel* mdl, const DevModel& hm, MpcBuffers& m, const MpcProblemDev& p, int b0, int b1, cudaStream_t stream, cudaEvent_t* ev) {
+int mpc_solve_launch(const DevModel* mdl, const DevModel& hm, MpcBuffers& m, const MpcProblemDev& p, int b0, int b1, cudaStream_t stream, cudaEvent_t* ev, bool value_fn) {
   const int nb = b1 - b0, nmax = m.nmax; if (nb <= 0) return 0;
   MpcSolutionDev prev = m.sol[m.cur], next = m.sol[1 - m.cur];   // the caller flips m.cur once all ranges are queued
   if (ev) cudaEventRecord(ev[0], stream);
@@ -1226,7 +1279,8 @@ int mpc_solve_launch(const DevModel* mdl, const DevModel& hm, MpcBuffers& m, con
     if (ev && it == iters - 1) cudaEventRecord(ev[7], stream);
     mpc_lq_kernel<<<(unsigned)((nodes + LQ_WARPS - 1) / LQ_WARPS), 32 * LQ_WARPS, sizeof(LqSmem) * LQ_WARPS, stream>>>(mdl, b0, b1, nmax, p, next, m.node_rec, m.stage, m.status);
     if (ev && it == iters - 1) cudaEventRecord(ev[2], stream);
-    mpc_riccati_kernel<<<nb, RIC_THREADS, sizeof(RicSmem), stream>>>(mdl, b0, b1, nmax, p, next, m.stage, m.gains, m.dx, m.du, m.robot, m.status);
+    if (value_fn && m.vf) mpc_riccati_kernel<true><<<nb, RIC_THREADS, sizeof(RicSmem), stream>>>(mdl, b0, b1, nmax, p, next, m.stage, m.gains, m.dx, m.du, m.robot, m.status, m.vf);
+    else mpc_riccati_kernel<false><<<nb, RIC_THREADS, sizeof(RicSmem), stream>>>(mdl, b0, b1, nmax, p, next, m.stage, m.gains, m.dx, m.du, m.robot, m.status, nullptr);
     if (ev && it == iters - 1) cudaEventRecord(ev[3], stream);
     if (ddp) { mpc_rollout_trials_kernel<<<(nb + ro_rpc - 1) / ro_rpc, ro_rpc * tr_pitch, (size_t)ro_rpc * GAIN_DBL * 8, stream>>>(mdl, b0, b1, nmax, p, next, m.stage, m.gains, m.ddp_trial, m.robot, m.status, n_trials, tr_pitch, ro_rpc);   // all step lengths side by side
       mpc_rollout_kernel<<<ro_grid, RO_THREADS, 0, stream>>>(mdl, b0, b1, nmax, p, next, m.stage, m.gains, m.ddp_trial, m.robot, m.status, m.step_info, 2, n_trials, tr_pitch, it); ++launched; }   // decision + in-place rollout of the accepted step
@@ -1251,6 +1305,10 @@ int mpc_policy_launch(const DevModel* mdl, const MpcBuffers& m, bool feedback, c
 int mpc_controller_export_launch(const DevModel* mdl, const MpcBuffers& m, bool valid, int b0, int count, double* bias, double* gain, int32_t* feedback, cudaStream_t stream) {
   if (count <= 0) return 0;
   mpc_controller_export_kernel<<<dim3(count, m.nmax), 32, 0, stream>>>(mdl, b0, m.nmax, m.sol[m.cur], m.stage, m.gains, m.status, valid ? 1 : 0, bias, gain, feedback);
+  return 1;
+}
+int mpc_value_function_launch(const MpcBuffers& m, bool valid, const double* t, const double* x, double* dfdx, double* dfdxx, int32_t* valid_out, cudaStream_t stream) {
+  mpc_value_function_kernel<<<(m.B + VF_WARPS - 1) / VF_WARPS, 32 * VF_WARPS, 0, stream>>>(m.B, m.nmax, m.sol[m.cur], m.vf, m.status, (valid && m.vf) ? 1 : 0, t, x, dfdx, dfdxx, valid_out);
   return 1;
 }
 int mpc_fixup_launch(const MpcBuffers& m, cudaStream_t stream) { mpc_fixup_kernel<<<m.B, 32, 0, stream>>>(m.B, m.nmax, m.sol[m.cur]); return 1; }

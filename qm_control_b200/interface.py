@@ -217,6 +217,23 @@ class Solver:
     def mpc_get_controller_dev(self, b0, count, bias, gain, feedback, stream=None):
         self._chk(self.lib.qmb200_mpc_get_controller_dev(self.h, int(b0), int(count), _p(bias), _p(gain), _p(feedback), C.c_void_p(stream) if stream else None), "qmb200_mpc_get_controller_dev")
 
+    def mpc_set_value_function(self, on=True):
+        """createValueFunction: the solve keeps the Riccati cost-to-go of its last QP for value_function (include/qmb200.h).  Refused with the DDP solver."""
+        self._chk(self.lib.qmb200_mpc_set_value_function(self.h, 1 if on else 0), "qmb200_mpc_set_value_function")
+
+    def mpc_get_value_function(self):
+        v = C.c_int32(); self._chk(self.lib.qmb200_mpc_get_value_function(self.h, C.byref(v)), "qmb200_mpc_get_value_function"); return bool(v.value)
+
+    def value_function(self, t, x):
+        """getValueFunction(t, x) of every robot → dict(dfdx[B, 30], dfdxx[B, 30, 30], valid[B]); f is 0.  Zero where valid is 0."""
+        B = self.batch; t = _f64(t, (B,)); x = _f64(x, (B, NX))
+        out = dict(dfdx=np.empty((B, NX)), dfdxx=np.empty((B, NX, NX)), valid=np.empty(B, dtype=np.int32))
+        self._chk(self.lib.qmb200_value_function(self.h, _p(t), _p(x), _p(out["dfdx"]), _p(out["dfdxx"]), _p(out["valid"])), "qmb200_value_function")
+        return out
+
+    def value_function_dev(self, t, x, dfdx, dfdxx, valid, stream=None):
+        self._chk(self.lib.qmb200_value_function_dev(self.h, _p(t), _p(x), _p(dfdx), _p(dfdxx), _p(valid), C.c_void_p(stream) if stream else None), "qmb200_value_function_dev")
+
     def tick(self, prob, t_eval, rbd, period):
         B = self.batch; a = self._prob(prob); t_eval = _f64(t_eval, (B,)); rbd = _f64(rbd, (B, RBD)); period = _f64(period, (B,))
         cmd = np.empty((B, CMD)); status = np.empty(B, dtype=np.int32)

@@ -1,5 +1,7 @@
 """Python mirror of the MPC seam: ocs2::SqpMpc as QMController::setupMpc builds it (qm_controllers/src/QMController.cpp:286-306):
 one multiple-shooting SQP iteration per advanceMpc(), warm-started from the previous PrimalSolution."""
+import numpy as np
+
 from .interface import QMInterface, Solver
 
 
@@ -24,6 +26,15 @@ class SqpMpc:
         """MPC_MRT_Interface::evaluatePolicy(currentTime, currentState) → (optimizedState, optimizedInput, plannedMode).  Without a state the
         feed-forward policy is evaluated."""
         return self.solver.policy_eval(t) if x is None else self.solver.policy_eval_state(t, x)
+
+    def setValueFunction(self, on=True):
+        """createValueFunction: keep the value function of each solve's last QP."""
+        self.solver.mpc_set_value_function(on)
+
+    def getValueFunction(self, t, x):
+        """SqpSolver::getValueFunction(time, state) of every robot → dict(f[B] = 0, dfdx[B, 30], dfdxx[B, 30, 30], valid[B]) (see Solver.value_function)."""
+        v = self.solver.value_function(t, x); v["f"] = np.zeros(self.batch)
+        return v
 
     def getLinearController(self, b0=0, count=None):
         """ocs2::LinearController of the last solve: dict(timeStamp[count, NMAX], biasArray, gainArray, feedback) (see Solver.mpc_get_controller)."""
